@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the reference's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's result to DIR/*.npy
 
 Metric (BASELINE.json): "acquisition candidates/sec + suggest() ms at n=4096 d=32; 1/2/4/8 GPU".
 One STEP = one pass of the scoring hot path over one candidate batch: fused posterior (mu, sigma^2) + MACE
@@ -20,6 +21,11 @@ Extra keys: `parity` (mu / sigma / objectives / front of a 2368-candidate sample
 cores, N = 1), `guard_flagged_frac` (rows the precision guard re-contracted on the FP32 pipe), `dense_regime` (a second
 workload, n=4096 d=8, where most candidates sit inside the data and the guard fires), `suggest` (suggest() ms with the
 fit / scoring split), `roofline`, `cpu_baseline`.
+
+--dump-outputs DIR writes what the last timed step of the headline workload returned to its caller, the global Pareto
+front: DIR/front_ids.npy (global candidate row, float64), DIR/front_objectives.npy ([K, 3] LCB, -logEI, -logPI, float32)
+and DIR/front_mu_sigma.npy ([K, 2], float32).  All inputs are seeded, so two builds run with the same arguments can be
+compared output for output.  bench.py writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -36,6 +42,7 @@ import time
 import numpy as np
 import torch
 
+sys.dont_write_bytecode = True        # no __pycache__ in the (possibly read-only) source tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -239,6 +246,15 @@ def parity_sample(gp, X, yt, tau, kappa, dev):
                       "criteria 1e-4 (mu scale-relative, sigma relative; rows with sigma^2 < 0.02 s listed separately, cap 2e-4)"}
 
 
+def dump_outputs(out_dir, front):
+    """front = pareto.front_read(...) of the last timed step: (global ids, F [K, 3], (mu, sigma) [K, 2])."""
+    os.makedirs(out_dir, exist_ok=True)
+    gid, F, mu_sigma = front
+    np.save(os.path.join(out_dir, "front_ids.npy"), gid.numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "front_objectives.npy"), F.numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "front_mu_sigma.npy"), mu_sigma.numpy().astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -249,7 +265,12 @@ def main():
     ap.add_argument("--no-suggest", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-dense", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's Pareto front to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA path's result: use it with --impl b200")
     steps, warmup = args.steps, max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -313,7 +334,7 @@ def main():
         them); max over ranks.  pipelined=True (N > 1 device step, whose front exchange runs on a separate stream under the
         NEXT step's scoring): ONE event pair around all K steps, the stream made to wait for every step's merged front before
         the closing event, minus the flush durations (own events) -- so the exchange that is still in flight after the last
-        scoring kernel is inside the timed region."""
+        scoring kernel is inside the timed region.  Returns (ms, wall ms, what the last step returned)."""
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(k)]
         barrier()
         t0 = time.perf_counter()
@@ -329,11 +350,12 @@ def main():
             for o in outs:
                 front_wait(o)
             end.record()
+            last = outs[-1]
         else:
             for a, b in ev:
                 flush.fill_(1)
                 a.record()
-                fn()
+                last = fn()
                 b.record()
         barrier()
         wall = (time.perf_counter() - t0) * 1e3
@@ -343,7 +365,7 @@ def main():
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), wall
+        return float(t.item()), wall, last
 
     def run_workload(n, d, seed, m, k_steps, k_warm, profile, fn="hartmann6"):
         """fit on rank 0 (+ broadcast), then time the device step and the end-to-end step over m candidates per rank"""
@@ -387,7 +409,7 @@ def main():
         lib.hb_launch_count(1)
         if profile:
             lib.hb_profile_enable(1)
-        total_ms, wall_ms = timed(step_dev, k_steps, pipelined=world > 1)
+        total_ms, wall_ms, last_dev = timed(step_dev, k_steps, pipelined=world > 1)
         launches = int(lib.hb_launch_count(1))
         kms, kn = C.c_double(0), C.c_int32(0)
         if profile:
@@ -395,18 +417,20 @@ def main():
             lib.hb_profile_enable(0)
         gs = (C.c_uint64 * 2)()
         lib.hb_guard_stats(gs, 1)
-        e2e_ms, _ = timed(step_e2e, k_steps)
+        e2e_ms, _, _ = timed(step_e2e, k_steps)
         t_region1 = time.perf_counter()
-        front = front_read(step_dev())
+        front = front_read(last_dev)
         return dict(gp=gp, X=X, yt=yt, tau=tau, kappa=kappa, total_ms=total_ms, wall_ms=wall_ms, e2e_ms=e2e_ms, launches=launches,
                     kms=kms.value, kn=kn.value, guard_frac=(gs[1] / gs[0]) if gs[0] else 0.0, fit_ms=fit_ms, region=(t_region0, t_region1),
-                    front_size=int(front[0].numel()))
+                    front=front, front_size=int(front[0].numel()))
 
     m = args.m_per_gpu
     w = run_workload(N_OBS, DIM, 1234 + 5, m, steps, warmup, True)
     if rank == 0 and sampler.proc is not None:
         sampler.window(*w["region"])
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, w["front"])
     gp = w["gp"]
     ms_per_step = w["total_ms"] / steps
     value = world * m / (ms_per_step / 1e3)

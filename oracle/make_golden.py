@@ -1,12 +1,14 @@
-"""Generates the committed golden fixtures under tests/golden/ (run in the BUILD container only).
+"""Generates the committed golden fixtures under tests/golden/ (needs a copy of the reference HEBO at
+``oracle.ref_loader.REF_ROOT``; nothing else does).
 
     python -m oracle.make_golden
 
 Two kinds of vectors:
-  * ``ref_*.npz``  -- outputs of the REFERENCE's own code loaded by path from /root/reference
-    (HEBO/hebo/acquisitions/acq.py MACE.eval, HEBO/hebo/models/scalers.py) on seeded inputs.  These pin
-    the oracle's MACE / scaler restatements (tests/test_oracle.py) and the CUDA MACE epilogue
-    (tests/test_gpu_parity.py).
+  * ``ref_*.npz``  -- outputs of the REFERENCE's own code loaded by path (HEBO/hebo/acquisitions/acq.py
+    MACE.eval, models/scalers.py, models/nn/sgld.py pSGLD, models/nn/mono_layers/layers.py KumarWarp,
+    models/layers.py EmbTransform, design_space/*.py DesignSpace) on seeded inputs.  These pin the oracle's
+    restatements (tests/test_oracle.py, tests/test_oracle_emb.py), the host design space (tests/test_host.py)
+    and the CUDA MACE epilogue (tests/test_gpu_parity.py).
   * ``gp_*.npz``   -- fp64 outputs of the oracle's restatement of the gpytorch exact-GP maths (no gpytorch
     install exists to generate them from; "parity unpinned" at that boundary, see oracle/gp_oracle.py)
     for small seeded versions of the BASELINE configs: loss, gradient, 100-epoch pSGLD trajectory end
@@ -82,6 +84,112 @@ def gen_ref_scalers():
                         yt=ss.transform(y).numpy())
 
 
+def gen_ref_mace_seeded():
+    """The reference's MACE on one seeded batch, its xi drawn by the reference itself after torch.manual_seed(11)
+    (tests/test_oracle.py replays that draw for the oracle)."""
+    ref = ref_loader.load_reference()
+
+    class Dummy(ref.BaseModel):
+        def __init__(self, mu, var):
+            super().__init__(1, 0, 1)
+            self.mu, self.var = mu, var
+
+        def fit(self, *a):
+            pass
+
+        def predict(self, x, xe):
+            return self.mu.clone(), self.var.clone()
+
+        @property
+        def noise(self):
+            return torch.tensor([0.02])
+
+    torch.manual_seed(3)
+    mu, var = torch.randn(777, 1), torch.rand(777, 1) + 1e-3
+    acq = ref.MACE(Dummy(mu, var), best_y=np.float32(-0.3), kappa=2.9)
+    torch.manual_seed(11)
+    F = acq(torch.zeros(777, 1), None)
+    np.savez_compressed(os.path.join(OUT, "ref_mace_seeded.npz"), mu=mu.numpy(), var=var.numpy(), F=F.numpy(),
+                        par=np.array([-0.3, 2.9, 0.02], dtype=np.float64))
+
+
+def gen_ref_psgld():
+    """Parameters after each of 25 steps of the reference's pSGLD (models/nn/sgld.py, its unrelated imports stubbed) on
+    the loss sum_i ||a_i * p_i||^2 + sum cos(p_i), noise drawn by the reference after torch.manual_seed(100 + step)."""
+    mod = ref_loader.load_file("_hebo_ref_nn.sgld", "models/nn/sgld.py",
+                               stubs=[("_hebo_ref_nn", ()), ("_hebo_ref_nn.deep_ensemble", ("BaseNet", "DeepEnsemble")),
+                                      ("matplotlib", ()), ("matplotlib.pyplot", ())])
+    g = torch.Generator().manual_seed(0)
+    params = [torch.nn.Parameter(torch.randn(s, generator=g, dtype=torch.float64)) for s in [(1,), (), (1, 5)]]
+    A = [torch.rand(p.numel(), generator=g, dtype=torch.float64) + 0.5 for p in params]
+    p0 = torch.cat([p.detach().reshape(-1).clone() for p in params])
+    n, lr, steps = 40, 0.01, 25
+    opt = mod.pSGLD(params, lr=lr, factor=1.0 / n, pretrain_step=steps // 10)
+    traj = []
+    for ep in range(steps):
+        torch.manual_seed(100 + ep)
+        opt.zero_grad()
+        sum(((a * p.reshape(-1)) ** 2).sum() + torch.cos(p.reshape(-1)).sum() for a, p in zip(A, params)).backward()
+        opt.step()
+        traj.append(torch.cat([p.detach().reshape(-1) for p in params]))
+    np.savez_compressed(os.path.join(OUT, "ref_psgld.npz"), p0=p0.numpy(), A=torch.cat(A).numpy(),
+                        traj=torch.stack(traj).numpy(), par=np.array([n, lr, steps], dtype=np.float64))
+
+
+def gen_ref_kumar_warp():
+    """The reference's KumarWarp layer (models/nn/mono_layers/layers.py) at seeded raw exponents, on [-1, 1] inputs
+    mapped to [0, 1] and back."""
+    mod = ref_loader.load_file("_hebo_ref_mono_layers", "models/nn/mono_layers/layers.py")
+    d = 6
+    layer = mod.KumarWarp(d).double()
+    g = torch.Generator().manual_seed(1)
+    with torch.no_grad():
+        layer._a.copy_(torch.randn(d, generator=g, dtype=torch.float64))
+        layer._b.copy_(torch.randn(d, generator=g, dtype=torch.float64))
+    X = torch.rand(200, d, generator=g, dtype=torch.float64) * 2 - 1
+    X[0], X[1] = -1.0, 1.0                               # the clamp at eps / 1 - eps
+    out = 2.0 * layer((X + 1.0) * 0.5).detach() - 1.0
+    np.savez_compressed(os.path.join(OUT, "ref_kumar_warp.npz"), raw_a=layer._a.detach().numpy(),
+                        raw_b=layer._b.detach().numpy(), a=layer.a.detach().numpy(), b=layer.b.detach().numpy(),
+                        X=X.numpy(), out=out.numpy())
+
+
+def gen_ref_emb():
+    """The reference's EmbTransform (models/layers.py): default sizes, its randomly initialised tables, and its output
+    on seeded category indices."""
+    mod = ref_loader.load_file("_hebo_ref_layers", "models/layers.py")
+    nu = [4, 7, 2, 120]
+    torch.manual_seed(0)
+    tr = mod.EmbTransform(nu)
+    g = torch.Generator().manual_seed(0)
+    Xe = torch.stack([torch.randint(0, u, (33,), generator=g) for u in nu], 1)
+    tables = {f"table{i}": m.weight.detach().double().numpy() for i, m in enumerate(tr.emb)}
+    np.savez_compressed(os.path.join(OUT, "ref_emb.npz"), num_uniqs=np.array(nu), emb_sizes=np.array(tr.emb_sizes),
+                        num_out=tr.num_out, Xe=Xe.numpy(), out=tr(Xe).detach().double().numpy(), **tables)
+
+
+def gen_ref_design_space():
+    """The reference's DesignSpace on tests/test_host.py's SPEC: names, optimisation bounds, transform of a fixed frame
+    and inverse transform of this package's own transform of it (each column as str(value), and as float where it is
+    numeric)."""
+    import pandas as pd
+    from hebo_b200.space import DesignSpace
+    from tests.test_host import FRAME, SPEC
+    df = pd.DataFrame(FRAME)
+    ref = ref_loader.load_design_space()().parse(SPEC)
+    rc, re_ = ref.transform(df)
+    xc, xe = DesignSpace().parse(SPEC).transform(df)
+    rb = ref.inverse_transform(xc, xe)
+    cols = {}
+    for col in ref.para_names:
+        cols[f"inv_{col}_str"] = np.array([str(v) for v in rb[col].tolist()])
+        num = pd.to_numeric(rb[col], errors="coerce").to_numpy(dtype=np.float64)
+        cols[f"inv_{col}_num"] = num if np.isfinite(num).all() else np.zeros(0)
+    np.savez_compressed(os.path.join(OUT, "ref_design_space.npz"), xc=rc.numpy(), xe=re_.numpy(),
+                        para_names=np.array(ref.para_names), opt_lb=ref.opt_lb.double().numpy(),
+                        opt_ub=ref.opt_ub.double().numpy(), **cols)
+
+
 def gen_gp(name, fn, n, d, m, q, kind, seed, warp=False, hetero=False):
     X, y = O.synthetic_problem(fn, n, d, seed)
     X = X.float().double()
@@ -151,6 +259,11 @@ def main():
     os.makedirs(OUT, exist_ok=True)
     gen_ref_mace()
     gen_ref_scalers()
+    gen_ref_mace_seeded()
+    gen_ref_psgld()
+    gen_ref_kumar_warp()
+    gen_ref_emb()
+    gen_ref_design_space()
     gen_gp("c1_branin", "branin", 64, 2, 256, 1, "matern32", 1235)            # BASELINE config 1
     gen_gp("c2_ackley", "ackley", 160, 8, 384, 8, "matern52", 1236)           # config 2, reduced n/m
     gen_gp("c3_hartmann_warp", "hartmann6", 200, 32, 384, 8, "matern32", 1237, warp=True)   # config 3, reduced

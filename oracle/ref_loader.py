@@ -1,10 +1,8 @@
-"""Load the reference's real ``acq.py`` / ``scalers.py`` / ``base_model.py`` by path.
+"""Load the reference's real source files (``acq.py``, ``scalers.py``, ``base_model.py``, ...) by path.
 
-TEST INFRASTRUCTURE ONLY, and only usable in the build container: /root/reference does not exist
-on the GPU box, so nothing that runs there (``-m gpu`` tests, smoke(), bench.py) may call this.
-It is used by ``oracle/make_golden.py`` to generate committed fixtures and by the CPU test
-``tests/test_oracle.py`` (skipped when /root/reference is absent) to pin the oracle's MACE /
-scaler restatements against the reference's own code.
+TEST INFRASTRUCTURE ONLY: used by ``oracle/make_golden.py`` alone, to record the reference's own outputs as
+the fixtures under ``tests/golden/``.  The tests, smoke() and bench.py read those fixtures and never the
+reference sources, so the repository runs and tests without a copy of the reference.
 
 ``import hebo`` itself fails here (pymoo / gpytorch missing: evolution_optimizer.py:14, gp.py:14);
 the files below import only torch/numpy/sklearn and load unmodified under stub parent packages.
@@ -50,3 +48,37 @@ def load_reference():
                                TorchMinMaxScaler=scalers.TorchMinMaxScaler,
                                TorchStandardScaler=scalers.TorchStandardScaler)
     return ns
+
+
+def load_file(modname: str, relpath: str, stubs=()):
+    """Load one reference source file unmodified, with the parent modules it imports but does not use replaced by
+    stubs: ``stubs`` lists (module name, names of placeholder classes it must provide)."""
+    saved = {}
+    for name, attrs in stubs:
+        saved[name] = sys.modules.get(name)
+        m = types.ModuleType(name)
+        m.__path__ = []
+        for k in attrs:
+            setattr(m, k, type(k, (), {}))
+        sys.modules[name] = m
+    try:
+        return _load(modname, relpath)
+    finally:
+        for name, old in saved.items():
+            if old is None:
+                sys.modules.pop(name, None)
+            else:
+                sys.modules[name] = old
+
+
+def load_design_space():
+    """The reference's DesignSpace class (design_space/*.py, loaded as one package)."""
+    pkg = "_hebo_ref_ds"
+    if pkg not in sys.modules:
+        m = types.ModuleType(pkg)
+        m.__path__ = [os.path.join(REF_ROOT, "design_space")]
+        sys.modules[pkg] = m
+    for mod in ("param", "numeric_param", "integer_param", "pow_param", "categorical_param", "bool_param",
+                "pow_integer_param", "int_exponent_param", "step_int", "design_space"):
+        _load(f"{pkg}.{mod}", os.path.join("design_space", mod + ".py"))
+    return sys.modules[f"{pkg}.design_space"].DesignSpace

@@ -175,12 +175,14 @@ SPEC = [{"name": "lr", "type": "pow", "lb": 1e-4, "ub": 1e-1}, {"name": "n", "ty
         {"name": "e", "type": "int_exponent", "lb": 32, "ub": 1024, "base": 2},
         {"name": "s", "type": "step_int", "lb": 4, "ub": 16, "step": 4},
         {"name": "c", "type": "cat", "categories": ["a", "b", "c"]}, {"name": "x", "type": "num", "lb": -1, "ub": 2}]
+FRAME = {"lr": [1e-3, 1e-1], "n": [3, 9], "b": [True, False], "w": [16, 300], "e": [64, 1024], "s": [8, 16], "c": ["b", "a"],
+         "x": [0.5, -1.0]}
 
 
 def test_design_space_types_round_trip_like_the_reference():
     """hebo_b200.space against the semantics of HEBO/hebo/design_space/*.py (transform / inverse_transform / bounds / the
-    pymoo variable kind of evolution_optimizer.py:26-41), incl. a cross-check with the reference's own classes when
-    /root/reference is present."""
+    pymoo variable kind of evolution_optimizer.py:26-41), incl. a cross-check with what the reference's own classes
+    compute on the same spec (tests/golden/ref_design_space.npz)."""
     import pandas as pd
     from hebo_b200.space import DesignSpace
     sp = DesignSpace().parse(SPEC)
@@ -188,8 +190,7 @@ def test_design_space_types_round_trip_like_the_reference():
     assert sp.var_kinds == ["real", "int", "int", "real", "int", "int", "real", "choice"] and sp.num_uniqs == [3]
     assert torch.allclose(sp.opt_lb, torch.tensor([-4., 1., 0., 3., 5., 0., -1., 0.], dtype=torch.float64))
     assert torch.allclose(sp.opt_ub, torch.tensor([-1., 9., 1., 9., 10., 3., 2., 2.], dtype=torch.float64))
-    df = pd.DataFrame({"lr": [1e-3, 1e-1], "n": [3, 9], "b": [True, False], "w": [16, 300], "e": [64, 1024], "s": [8, 16],
-                       "c": ["b", "a"], "x": [0.5, -1.0]})
+    df = pd.DataFrame(FRAME)
     xc, xe = sp.transform(df)
     assert xc.dtype == torch.float32 and xe.dtype == torch.int64 and xe.reshape(-1).tolist() == [1, 0]
     assert torch.allclose(xc[0], torch.tensor([-3., 3., 1., 4., 6., 1., 0.5]))
@@ -202,22 +203,13 @@ def test_design_space_types_round_trip_like_the_reference():
     xs, es = sp.transform(smp)
     lo, hi = sp.opt_lb.float(), sp.opt_ub.float()
     assert bool(((torch.cat([xs, es.float()], 1) >= lo - 1e-5) & (torch.cat([xs, es.float()], 1) <= hi + 1e-5)).all())
-    ref_dir = "/root/reference/HEBO/hebo/design_space"
-    import os
-    if os.path.isdir(ref_dir):                       # the reference's own DesignSpace, loaded by path (build container only)
-        import importlib.util, sys, types
-        pkg = types.ModuleType("_ref_ds"); pkg.__path__ = [ref_dir]; sys.modules["_ref_ds"] = pkg
-        for mod in ("param", "numeric_param", "integer_param", "pow_param", "categorical_param", "bool_param", "pow_integer_param",
-                    "int_exponent_param", "step_int", "design_space"):
-            spec = importlib.util.spec_from_file_location(f"_ref_ds.{mod}", os.path.join(ref_dir, mod + ".py"))
-            m = importlib.util.module_from_spec(spec); sys.modules[f"_ref_ds.{mod}"] = m; spec.loader.exec_module(m)
-        ref = sys.modules["_ref_ds.design_space"].DesignSpace().parse(SPEC)
-        rc, re_ = ref.transform(df)
-        assert torch.allclose(rc, xc) and torch.equal(re_, xe) and ref.para_names == sp.para_names
-        assert torch.allclose(ref.opt_lb.double(), sp.opt_lb) and torch.allclose(ref.opt_ub.double(), sp.opt_ub)
-        rb = ref.inverse_transform(xc, xe)
-        for col in sp.para_names:
-            assert [str(v) for v in rb[col].tolist()] == [str(v) for v in back[col].tolist()] or np.allclose(rb[col].values.astype(float), back[col].values.astype(float))
+    ref = load_golden("ref_design_space.npz")                # the reference's own DesignSpace on SPEC / FRAME
+    assert torch.allclose(torch.from_numpy(ref["xc"]), xc) and torch.equal(torch.from_numpy(ref["xe"]), xe)
+    assert ref["para_names"].tolist() == sp.para_names
+    assert torch.allclose(torch.from_numpy(ref["opt_lb"]), sp.opt_lb) and torch.allclose(torch.from_numpy(ref["opt_ub"]), sp.opt_ub)
+    for col in sp.para_names:
+        rb_str, rb_num = ref[f"inv_{col}_str"].tolist(), ref[f"inv_{col}_num"]
+        assert rb_str == [str(v) for v in back[col].tolist()] or (rb_num.size and np.allclose(rb_num, back[col].values.astype(float)))
 
 
 def test_standalone_hebo_host_logic_typed_space():

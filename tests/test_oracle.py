@@ -1,5 +1,5 @@
-"""CPU tests: the oracle against the committed golden vectors (and, when /root/reference is mounted,
-against the reference's own acq.py / scalers.py loaded by path)."""
+"""CPU tests: the oracle against the committed golden vectors, among them the outputs of the reference's own
+acq.py / scalers.py / sgld.py / KumarWarp recorded by oracle/make_golden.py."""
 import math
 
 import numpy as np
@@ -7,7 +7,6 @@ import pytest
 import torch
 
 from oracle import gp_oracle as O
-from oracle import ref_loader
 from tests.util import load_golden
 
 GP_CASES = ["c1_branin", "c2_ackley", "c3_hartmann_warp", "c4_hetero", "rbf"]
@@ -43,33 +42,15 @@ def test_scaler_restatement_matches_reference_vectors():
     np.testing.assert_allclose(std, g["std"], rtol=1e-6)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_mace_live_against_reference_source():
-    ref = ref_loader.load_reference()
-
-    class Dummy(ref.BaseModel):
-        def __init__(self, mu, var):
-            super().__init__(1, 0, 1)
-            self.mu, self.var = mu, var
-
-        def fit(self, *a):
-            pass
-
-        def predict(self, x, xe):
-            return self.mu.clone(), self.var.clone()
-
-        @property
-        def noise(self):
-            return torch.tensor([0.02])
-
-    torch.manual_seed(3)
-    mu, var = torch.randn(777, 1), torch.rand(777, 1) + 1e-3
-    acq = ref.MACE(Dummy(mu, var), best_y=np.float32(-0.3), kappa=2.9)
-    torch.manual_seed(11)
-    Fr = acq(torch.zeros(777, 1), None)
+    """The reference's MACE on a seeded batch (tests/golden/ref_mace_seeded.npz), its xi drawn by the reference itself
+    after torch.manual_seed(11): the oracle, given the same draws in the same order, reproduces its objectives."""
+    g = load_golden("ref_mace_seeded.npz")
+    mu, var, Fr = torch.from_numpy(g["mu"]), torch.from_numpy(g["var"]), torch.from_numpy(g["F"])
+    best_y, kappa, noise = g["par"]
     torch.manual_seed(11)
     xi1, xi2 = torch.randn(777, 1), torch.randn(777, 1)
-    F = O.mace(mu, var, 0.02, float(np.float32(-0.3)), 2.9, 1e-4, xi1, xi2)
+    F = O.mace(mu, var, float(noise), float(np.float32(best_y)), float(kappa), 1e-4, xi1, xi2)
     # not bit-equal: the reference gathers rows before log() (acq.py:169-170), which changes ATen's
     # vector/scalar-tail split and with it the last ulps of erf/exp/log
     torch.testing.assert_close(F, Fr, rtol=2e-4, atol=2e-4)
@@ -166,59 +147,22 @@ def test_kappa_schedule_and_lengthscale_init():
     assert abs(float(ls[0]) - float(torch.pdist(X).median())) < 1e-15
 
 
-def _load_ref_file(modname, relpath, stubs=()):
-    """Load one reference source file unmodified under stub parents (build container only)."""
-    import importlib.util
-    import sys
-    import types
-    saved = {}
-    for name, attrs in stubs:
-        saved[name] = sys.modules.get(name)
-        m = types.ModuleType(name)
-        m.__path__ = []
-        for k in attrs:
-            setattr(m, k, type(k, (), {}))
-        sys.modules[name] = m
-    try:
-        spec = importlib.util.spec_from_file_location(modname, "/root/reference/HEBO/hebo/" + relpath,
-                                                      submodule_search_locations=None)
-        mod = importlib.util.module_from_spec(spec)
-        sys.modules[modname] = mod
-        spec.loader.exec_module(mod)
-        return mod
-    finally:
-        for name, old in saved.items():
-            if old is None:
-                sys.modules.pop(name, None)
-            else:
-                sys.modules[name] = old
-
-
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_psgld_step_against_the_reference_optimizer_class():
-    """oracle.psgld_step vs the reference's real pSGLD (HEBO/hebo/models/nn/sgld.py:49-70, loaded unmodified; its
-    unrelated imports -- deep_ensemble, matplotlib -- are stubbed): same parameters after 25 steps over three parameter
-    tensors with the reference's own torch.randn_like draws replayed as the oracle's xi."""
-    mod = _load_ref_file("_hebo_ref_nn.sgld", "models/nn/sgld.py",
-                         stubs=[("_hebo_ref_nn", ()), ("_hebo_ref_nn.deep_ensemble", ("BaseNet", "DeepEnsemble")),
-                                ("matplotlib", ()), ("matplotlib.pyplot", ())])
-    g = torch.Generator().manual_seed(0)
+    """oracle.psgld_step vs the reference's real pSGLD (HEBO/hebo/models/nn/sgld.py:49-70; its parameters after each
+    step are in tests/golden/ref_psgld.npz): same parameters after 25 steps over three parameter tensors with the
+    reference's own torch.randn_like draws replayed as the oracle's xi."""
+    ref = load_golden("ref_psgld.npz")
     shapes = [(1,), (), (1, 5)]
-    params = [torch.nn.Parameter(torch.randn(s, generator=g, dtype=torch.float64)) for s in shapes]
-    A = [torch.rand(p.numel(), generator=g, dtype=torch.float64) + 0.5 for p in params]
+    A = torch.from_numpy(ref["A"]).split([int(np.prod(s)) for s in shapes])
+    vec = torch.from_numpy(ref["p0"])
 
     def loss_of(ps):                # a smooth non-quadratic test loss
         return sum(((a * p.reshape(-1)) ** 2).sum() + torch.cos(p.reshape(-1)).sum() for a, p in zip(A, ps))
-    n, lr, steps = 40, 0.01, 25
-    opt = mod.pSGLD(params, lr=lr, factor=1.0 / n, pretrain_step=steps // 10)
-    vec = torch.cat([p.detach().reshape(-1).clone() for p in params])
+    n, lr, steps = ref["par"]
+    n, steps = int(n), int(steps)
+    assert ref["traj"].shape == (steps, vec.numel())
     st = O.PSGLDState(torch.zeros_like(vec))
     for ep in range(steps):
-        # reference step (draws from the global generator, in parameter order, after the pretrain phase)
-        torch.manual_seed(100 + ep)
-        opt.zero_grad()
-        loss_of(params).backward()
-        opt.step()
         # oracle step with the same draws
         torch.manual_seed(100 + ep)
         xi = None
@@ -231,26 +175,21 @@ def test_psgld_step_against_the_reference_optimizer_class():
             ps.append(v[off:off + k].reshape(s))
             off += k
         (gr,) = torch.autograd.grad(loss_of(ps), v)
-        vec = O.psgld_step(vec, gr, st, lr, 1.0 / n, steps // 10, xi)
-        ref_vec = torch.cat([p.detach().reshape(-1) for p in params])
+        vec = O.psgld_step(vec, gr, st, float(lr), 1.0 / n, steps // 10, xi)
+        ref_vec = torch.from_numpy(ref["traj"][ep])
         assert float((vec - ref_vec).abs().max()) < 1e-13, ep
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted (GPU box)")
 def test_kumaraswamy_warp_against_the_reference_layer():
-    """oracle.warp_oracle.warp / exponents vs the reference's KumarWarp layer (mono_layers/layers.py:85-117, loaded
-    unmodified): a, b = 0.01 + 9.99 sigmoid(raw), w(u) = 1 - (1 - clamp(u)^a)^b on u = (x + 1) / 2."""
+    """oracle.warp_oracle.warp / exponents vs the reference's KumarWarp layer (mono_layers/layers.py:85-117; its exponents
+    and outputs are in tests/golden/ref_kumar_warp.npz): a, b = 0.01 + 9.99 sigmoid(raw), w(u) = 1 - (1 - clamp(u)^a)^b on
+    u = (x + 1) / 2."""
     from oracle import warp_oracle as W
-    mod = _load_ref_file("_hebo_ref_mono_layers", "models/nn/mono_layers/layers.py")
-    d = 6
-    layer = mod.KumarWarp(d).double()
-    g = torch.Generator().manual_seed(1)
-    with torch.no_grad():
-        layer._a.copy_(torch.randn(d, generator=g, dtype=torch.float64))
-        layer._b.copy_(torch.randn(d, generator=g, dtype=torch.float64))
-    assert torch.equal(W.exponents(layer._a.detach()), layer.a.detach())
-    X = torch.rand(200, d, generator=g, dtype=torch.float64) * 2 - 1
-    X[0], X[1] = -1.0, 1.0                               # the clamp at eps / 1 - eps
-    ours = W.warp(X, layer.a.detach(), layer.b.detach())
-    ref = 2.0 * layer((X + 1.0) * 0.5).detach() - 1.0
-    assert float((ours - ref).abs().max()) < 1e-15
+    ref = load_golden("ref_kumar_warp.npz")
+    a, b = torch.from_numpy(ref["a"]), torch.from_numpy(ref["b"])
+    assert torch.equal(W.exponents(torch.from_numpy(ref["raw_a"])), a)
+    assert torch.equal(W.exponents(torch.from_numpy(ref["raw_b"])), b)
+    X = torch.from_numpy(ref["X"])
+    assert float(X.min()) == -1.0 and float(X.max()) == 1.0          # the clamp at eps / 1 - eps is exercised
+    ours = W.warp(X, a, b)
+    assert float((ours - torch.from_numpy(ref["out"])).abs().max()) < 1e-15

@@ -2,6 +2,7 @@
 import torch
 
 from oracle import emb_oracle as E
+from tests.util import load_golden
 
 
 def problem(n=60, d=3, num_uniqs=(4, 7), seed=0):
@@ -58,24 +59,13 @@ def test_unused_categories_get_zero_gradient_and_prediction_is_consistent():
 
 
 def test_embedding_lookup_matches_the_reference_module():
-    """Pins `embed` against the reference's real EmbTransform (HEBO/hebo/models/layers.py:14-34, loaded by path; build
-    container only): same default sizes, same column order, same concatenation."""
-    import importlib.util
-    import os
-    import pytest
-    path = "/root/reference/HEBO/hebo/models/layers.py"
-    if not os.path.isfile(path):
-        pytest.skip("/root/reference is not present")
-    spec = importlib.util.spec_from_file_location("_hebo_ref_layers", path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    nu = [4, 7, 2, 120]
-    tr = mod.EmbTransform(nu)
-    assert tr.emb_sizes == E.default_emb_sizes(nu) and tr.num_out == sum(E.default_emb_sizes(nu))
-    g = torch.Generator().manual_seed(0)
-    Xe = torch.stack([torch.randint(0, u, (33,), generator=g) for u in nu], 1)
-    tables = [m.weight.detach().double() for m in tr.emb]
-    assert torch.equal(E.embed(Xe, tables), tr(Xe).detach().double())
+    """Pins `embed` against the reference's real EmbTransform (HEBO/hebo/models/layers.py:14-34; its sizes, tables and
+    output are in tests/golden/ref_emb.npz): same default sizes, same column order, same concatenation."""
+    ref = load_golden("ref_emb.npz")
+    nu = ref["num_uniqs"].tolist()
+    assert ref["emb_sizes"].tolist() == E.default_emb_sizes(nu) and int(ref["num_out"]) == sum(E.default_emb_sizes(nu))
+    tables = [torch.from_numpy(ref[f"table{i}"]) for i in range(len(nu))]
+    assert torch.equal(E.embed(torch.from_numpy(ref["Xe"]), tables), torch.from_numpy(ref["out"]))
 
 
 def test_general_layouts_closed_form_vs_autograd():
