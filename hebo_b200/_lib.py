@@ -82,10 +82,13 @@ SIGNATURES = {
     "hb_sample_y": (_i32, [_vp, _vp, _i64, _i64, _i64, _sp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _f32, _f32, _i32, _vp, _i32,
                            _vp, C.POINTER(C.c_float), _vp, _i64, _vp]),
     "hb_mace_epilogue": (_i32, [_vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp, _vp, _u64, _vp, _vp]),
+    "hb_general_acq_epilogue": (_i32, [_vp, _vp, _i64, _i32, _i32, _vp, _f32, _f32, _i32, _vp, _u64, _i64, _vp, _vp, _vp]),
+    "hb_pareto_front": (_i32, [_vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _i64, _vp]),
     "hb_pareto_front3": (_i32, [_vp, _i64, _vp, _vp, _vp, _i64, _vp]),
     "hb_nsga2_init": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _u64, _vp, _vp, _vp]),
     "hb_nsga2_mate": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _u64, _i32, _vp, _vp, _vp, _vp]),
     "hb_nsga2_survive": (_i32, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "hb_nsga2_survive_k": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hb_front_merge_workspace_bytes": (_i64, [_i64, _i64]),
     "hb_front_pack": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp]),
     "hb_front_merge": (_i32, [_vp, _i64, _i64, _vp, _vp, _i64, _vp]),

@@ -3,7 +3,9 @@
 ``MACE`` is the drop-in for the reference's MACE (acq.py:131-171): with a ``hebo_b200.GP`` model the
 predict + (LCB, -logEI, -logPI) arithmetic is ONE fused C-ABI call (``GP.predict_mace``); with any other
 ``BaseModel`` that model's ``predict`` output is pushed through the same CUDA epilogue (``hb_mace_epilogue``), so the
-class stays a valid general-purpose acquisition.  ``Mean`` / ``Sigma`` / ``LCB`` mirror acq.py:55-82.
+class stays a valid general-purpose acquisition.  ``GeneralAcq`` (acq.py:192-242: LCB of every objective and constraint
+output, the acquisition of ``GeneralBO``) follows the same pattern with ``hb_general_acq_epilogue``.  ``Mean`` / ``Sigma`` /
+``LCB`` mirror acq.py:55-82.
 """
 from __future__ import annotations
 
@@ -11,7 +13,7 @@ import numpy as np
 import torch
 
 from .base import Acquisition
-from .gp import GP
+from .gp import GP, MultiTaskModel
 
 
 class SingleObjectiveAcq(Acquisition):
@@ -99,6 +101,85 @@ class MACE(Acquisition):
                                                        float(self.kappa), float(self.eps), _lib.ptr(z1), _lib.ptr(z2), 0, _lib.ptr(F),
                                                        _lib.stream_ptr()), "hb_mace_epilogue")
         return F.cpu()
+
+
+class GeneralAcq(Acquisition):
+    """Constrained multi-objective LCB (acq.py:192-242): minimise (lcb_o1, ..., lcb_oK) subject to lcb_c1 < 0, ...
+
+    out[:, :num_obj] = py - kappa ps and out[:, num_obj:] = py - c_kappa ps, with py += sqrt(noise) xi when use_noise.
+    With a ``hebo_b200.MultiTaskModel`` (or a single-output ``GP`` when O = 1) the O per-output posteriors are enqueued back
+    to back into one [O, m] device buffer and the CUDA epilogue follows, with no host synchronisation in between (each
+    output's failed-fit degradation, gp.py:152-154, stays in its own posterior); with any other ``BaseModel`` its
+    ``predict`` output goes through the same epilogue.  xi: one torch.randn(m, O) from torch's CPU generator after predict,
+    like the reference, when the model's rng is 'host'; in-kernel Philox normals otherwise."""
+
+    def __init__(self, model, num_obj, num_constr, **conf):
+        super().__init__(model, **conf)
+        self._num_obj = num_obj
+        self._num_constr = num_constr
+        self.kappa = conf.get("kappa", 2.0)
+        self.c_kappa = conf.get("c_kappa", 0.)
+        self.use_noise = conf.get("use_noise", True)
+        assert self.model.num_out == self.num_obj + self.num_constr
+        assert self.num_obj >= 1
+
+    @property
+    def num_obj(self) -> int:
+        return self._num_obj
+
+    @property
+    def num_constr(self) -> int:
+        return self._num_constr
+
+    def eval(self, x, xe=None):
+        return self.evaluate(x, xe)
+
+    def _device_models(self):
+        if isinstance(self.model, MultiTaskModel) and all(isinstance(g, GP) for g in self.model.models):
+            return self.model.models
+        if isinstance(self.model, GP) and self.model.num_out == 1:
+            return [self.model]
+        return None
+
+    def evaluate(self, x, xe=None, device_out: bool = False, return_cv: bool = False, seed: int = 0):
+        """out [m, O] (and cv [m] = sum_j max(0, out[:, num_obj + j]) with return_cv) on the input's device, or on the GPU
+        with device_out=True.  seed keys the Philox draws of the 'device' rng."""
+        from . import _lib
+        O, K = self.num_obj + self.num_constr, self.num_obj
+        gps = self._device_models()
+        with torch.no_grad():
+            if gps is not None:
+                g0 = gps[0]
+                dev = g0.device
+                m = g0._rows(x, xe)
+                on_cpu = not device_out and not any(torch.is_tensor(t) and t.is_cuda for t in (x, xe))
+                mu = torch.empty(O, m, dtype=torch.float32, device=dev)
+                var = torch.empty(O, m, dtype=torch.float32, device=dev)
+                if m:
+                    Xs, xe_dev = g0._to_dev(x), g0._xe_dev(xe, m)
+                    for o, g in enumerate(gps):
+                        g._posterior(Xs, False, Xe_dev=xe_dev, out_mu=mu[o], out_var=var[o])
+                host_rng = g0.rng == "host"
+            else:
+                dev = torch.device("cuda")
+                on_cpu = not device_out and not (torch.is_tensor(x) and x.is_cuda)
+                py, ps2 = self.model.predict(x, xe)
+                m = py.shape[0]
+                mu = py.reshape(m, O).t().to(dev, torch.float32).contiguous()
+                var = ps2.reshape(m, O).t().to(dev, torch.float32).contiguous()
+                host_rng = True
+            noise = torch.as_tensor(self.model.noise, dtype=torch.float32).reshape(-1).to(dev).contiguous() if self.use_noise else None
+            xi = torch.randn(m, O).to(dev).contiguous() if (self.use_noise and host_rng) else None   # acq.py:238
+            out = torch.empty(m, O, dtype=torch.float32, device=dev)
+            cv = torch.empty(m, dtype=torch.float32, device=dev)
+            if m:
+                with torch.cuda.device(dev):
+                    _lib.check(_lib.lib().hb_general_acq_epilogue(_lib.ptr(mu), _lib.ptr(var), m, K, O - K, _lib.ptr(noise), float(self.kappa),
+                                                                  float(self.c_kappa), int(bool(self.use_noise)), _lib.ptr(xi), int(seed), 0,
+                                                                  _lib.ptr(out), _lib.ptr(cv), _lib.stream_ptr()), "hb_general_acq_epilogue")
+        if on_cpu:
+            out, cv = out.cpu(), cv.cpu()
+        return (out, cv) if return_cv else out
 
 
 FusedMACE = MACE

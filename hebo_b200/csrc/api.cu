@@ -757,6 +757,20 @@ int32_t hb_mace_epilogue(const float *mu, const float *var, int64_t m, float noi
   return launch_mace_only(mu, var, m, noise_var, tau, kappa, eps, xi1, xi2, seed, F, (cudaStream_t)stream);
 }
 
+int32_t hb_general_acq_epilogue(const float *mu, const float *var, int64_t m, int32_t num_obj, int32_t num_constr,
+                                const float *noise_var, float kappa, float c_kappa, int32_t use_noise, const float *xi, uint64_t seed,
+                                int64_t rng_offset, float *out, float *cv, void *stream) {
+  if (!mu || !var || !out || (use_noise && !noise_var)) return HB_ERR_INVALID;
+  return launch_general_acq(mu, var, m, num_obj, num_constr, noise_var, kappa, c_kappa, use_noise, xi, seed, rng_offset, out, cv,
+                            (cudaStream_t)stream);
+}
+
+int32_t hb_pareto_front(const float *F, int64_t m, int32_t K, int64_t ldf, const float *cv, int32_t *idx_out, int32_t *count,
+                        void *ws, int64_t ws_bytes, void *stream) {
+  if (!F || !idx_out || !count || !ws || K < 1 || K > 8 || ldf < K) return HB_ERR_INVALID;
+  return launch_pareto(F, m, K, ldf, cv, idx_out, count, ws, ws_bytes, (cudaStream_t)stream);
+}
+
 int32_t hb_pareto_front3(const float *F, int64_t m, int32_t *idx_out, int32_t *count, void *ws, int64_t ws_bytes,
                          void *stream) {
   if (!F || !idx_out || !count || !ws) return HB_ERR_INVALID;
@@ -796,6 +810,14 @@ int32_t hb_nsga2_survive(const float *X, const float *F, const float *C, const f
                          float *X_next, float *F_next, float *Xc_next, int32_t *Xe_next, void *stream) {
   if (!X || !F || !C || !FC || !X_next || !F_next || (d > 0 && !Xc_next) || (D > d && !Xe_next)) return HB_ERR_INVALID;
   return launch_nsga_survive(X, F, C, FC, pop, D, d, X_next, F_next, Xc_next, Xe_next, (cudaStream_t)stream);
+}
+
+int32_t hb_nsga2_survive_k(const float *X, const float *F, const float *CV, const float *C, const float *FC, const float *CVC,
+                           int64_t pop, int64_t D, int64_t d, int32_t K, float *X_next, float *F_next, float *CV_next,
+                           float *Xc_next, int32_t *Xe_next, void *stream) {
+  if (!X || !F || !C || !FC || !X_next || !F_next || (d > 0 && !Xc_next) || (D > d && !Xe_next)) return HB_ERR_INVALID;
+  if (K < 1 || K > 8 || (CV == nullptr) != (CVC == nullptr) || (CV && !CV_next)) return HB_ERR_INVALID;
+  return launch_nsga_survive_k(X, F, CV, C, FC, CVC, pop, D, d, K, X_next, F_next, CV_next, Xc_next, Xe_next, (cudaStream_t)stream);
 }
 
 }  // extern "C"

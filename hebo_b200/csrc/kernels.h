@@ -92,6 +92,9 @@ size_t posterior_ws_bytes(int64_t np, int64_t d, int64_t m_chunk);
 int guard_stats(unsigned long long *out, int reset);
 int launch_mace_only(const float *mu, const float *var, int64_t m, float noise_var, float tau, float kappa, float eps,
                      const float *xi1, const float *xi2, uint64_t seed, float *F, cudaStream_t st);
+int launch_general_acq(const float *mu, const float *var, int64_t m, int num_obj, int num_constr, const float *noise_var,
+                       float kappa, float c_kappa, int use_noise, const float *xi, uint64_t seed, int64_t rng_offset, float *out,
+                       float *cv, cudaStream_t st);
 
 // fp16 two-level split tensor path of the posterior (vnorm_h16.cu: tcgen05 / TMEM / TMA)
 int kstar_groups(int64_t np);
@@ -110,6 +113,8 @@ int launch_vnorm_h16(const __half *ks_h0, const __half *ks_h1, int64_t ks_rows, 
                      cudaStream_t st);
 
 // pareto.cu
+int launch_pareto(const float *F, int64_t m, int K, int64_t ldf, const float *cv, int32_t *idx_out, int32_t *count, void *ws,
+                  int64_t ws_bytes, cudaStream_t st);
 int launch_pareto3(const float *F, int64_t m, int32_t *idx_out, int32_t *count, void *ws, int64_t ws_bytes,
                    cudaStream_t st);
 size_t pareto_ws_bytes(int64_t m);
@@ -131,5 +136,8 @@ int launch_nsga_mate(const float *X, int64_t P, int64_t D, int64_t d, const int3
                      const float *fixed, uint64_t seed, int gen, float *C, float *Cc, int32_t *Ce, cudaStream_t st);
 int launch_nsga_survive(const float *X, const float *F, const float *C, const float *FC, int64_t P, int64_t D, int64_t d,
                         float *Xn, float *Fn, float *Xcn, int32_t *Xen, cudaStream_t st);
+int launch_nsga_survive_k(const float *X, const float *F, const float *CV, const float *C, const float *FC, const float *CVC,
+                          int64_t P, int64_t D, int64_t d, int K, float *Xn, float *Fn, float *CVn, float *Xcn, int32_t *Xen,
+                          cudaStream_t st);
 
 }  // namespace hb

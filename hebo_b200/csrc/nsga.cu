@@ -127,26 +127,41 @@ __global__ void nsga_mate_kernel(const float *__restrict__ X, int P, int D, int 
   if (second) split_row(c2, d, D - d, Cc + (int64_t)(2 * t + 1) * d, Ce + (int64_t)(2 * t + 1) * (D - d));
 }
 
-// ---- rank-and-crowding survival of the merged population (pop rows 0..P-1, offspring rows P..2P-1), one CTA.
+// ---- rank-and-crowding survival of the merged population (pop rows 0..P-1, offspring rows P..2P-1), one CTA, K objectives.
+// Without constraints (CV == nullptr) every row takes part; a non-finite objective becomes +inf and a duplicate child
+// all +inf, so they only fill slots nothing else can.  With constraints (CV / CVC [P] = sum_j max(0, g_j), pymoo 0.6 calc_cv
+// as recalled; evolution_optimizer.py:104-105 hands pymoo F and G) the filter_infeasible rule of pymoo's Survival.do:
+// the feasible rows (cv <= 0, finite objectives, not a duplicate) go through rank-and-crowding for min(n_feasible, P) slots,
+// the remaining slots go to the other rows in ascending cv (lower merged index first on ties), duplicates and rows with a
+// non-finite objective or a NaN cv last.
 constexpr int NSGA_MAX = 512;
+template <int K>
 __global__ void __launch_bounds__(NSGA_MAX) nsga_survive_kernel(const float *__restrict__ X, const float *__restrict__ F,
-                                                                const float *__restrict__ C, const float *__restrict__ FC,
+                                                                const float *__restrict__ CV, const float *__restrict__ C,
+                                                                const float *__restrict__ FC, const float *__restrict__ CVC,
                                                                 int P, int D, int d, float *__restrict__ Xn,
-                                                                float *__restrict__ Fn, float *__restrict__ Xcn,
-                                                                int32_t *__restrict__ Xen) {
-  __shared__ float f[NSGA_MAX][3];
+                                                                float *__restrict__ Fn, float *__restrict__ CVn,
+                                                                float *__restrict__ Xcn, int32_t *__restrict__ Xen) {
+  __shared__ float f[NSGA_MAX][K];
   __shared__ int ndom[NSGA_MAX], rank[NSGA_MAX], order[NSGA_MAX];
-  __shared__ float crowd[NSGA_MAX];
-  __shared__ unsigned char infront[NSGA_MAX], keep[NSGA_MAX];
-  __shared__ int cnt, cum, r_cut, need;
+  __shared__ float crowd[NSGA_MAX], cvk[NSGA_MAX];
+  __shared__ unsigned char infront[NSGA_MAX], keep[NSGA_MAX], part[NSGA_MAX], bad[NSGA_MAX];
+  __shared__ int cnt, cum, r_cut, need, nfeas;
   const int N = 2 * P, i = threadIdx.x;
   const bool on = i < N;
+  const bool constrained = CV != nullptr;
+  if (i == 0) nfeas = 0;
   if (on) {
-    const float *src = i < P ? F + (int64_t)i * 3 : FC + (int64_t)(i - P) * 3;
-    for (int k = 0; k < 3; ++k) {
+    const float *src = i < P ? F + (int64_t)i * K : FC + (int64_t)(i - P) * K;
+    bool finite = true;
+    for (int k = 0; k < K; ++k) {
       const float v = src[k];
+      finite &= isfinite(v);
       f[i][k] = isfinite(v) ? v : INFINITY;                // NaN / inf objectives never survive (evolution_optimizer.py:104 F)
     }
+    const float c = constrained ? (i < P ? CV[i] : CVC[i - P]) : 0.0f;
+    bad[i] = constrained && (!finite || isnan(c));
+    cvk[i] = bad[i] ? 0.0f : c;
     rank[i] = -1;
     keep[i] = 0;
     infront[i] = 0;
@@ -163,25 +178,42 @@ __global__ void __launch_bounds__(NSGA_MAX) nsga_survive_kernel(const float *__r
       for (int k = 0; k < D && same; ++k) same = fabsf(o[k] - me[k]) <= 1e-16f;
       dup = same;
     }
-    if (dup) f[i][0] = f[i][1] = f[i][2] = INFINITY;
+    if (dup) {
+      for (int k = 0; k < K; ++k) f[i][k] = INFINITY;
+      if (constrained) {
+        bad[i] = 1;
+        cvk[i] = 0.0f;
+      }
+    }
   }
   __syncthreads();
   if (on) {
-    int c = 0;
-    for (int j = 0; j < N; ++j) {
-      const bool le = f[j][0] <= f[i][0] && f[j][1] <= f[i][1] && f[j][2] <= f[i][2];
-      const bool lt = f[j][0] < f[i][0] || f[j][1] < f[i][1] || f[j][2] < f[i][2];
-      c += (le && lt) ? 1 : 0;
+    part[i] = !constrained || (!bad[i] && cvk[i] <= 0.0f);
+    if (constrained && part[i]) atomicAdd(&nfeas, 1);
+  }
+  __syncthreads();
+  const int Pf = constrained ? min(nfeas, P) : P;          // slots filled by rank-and-crowding
+  auto dominates = [&](int j) {
+    bool le = true, lt = false;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      le = le && f[j][k] <= f[i][k];
+      lt = lt || f[j][k] < f[i][k];
     }
+    return le && lt;
+  };
+  if (on && part[i]) {
+    int c = 0;
+    for (int j = 0; j < N; ++j) c += (part[j] && dominates(j)) ? 1 : 0;
     ndom[i] = c;
   }
   if (i == 0) { cum = 0; r_cut = -1; need = 0; }
   __syncthreads();
-  // ---- front peeling until P survivors are covered
-  for (int r = 0; r < N; ++r) {
+  // ---- front peeling until Pf survivors are covered
+  for (int r = 0; r < N && Pf > 0; ++r) {
     if (i == 0) cnt = 0;
     __syncthreads();
-    if (on && rank[i] < 0 && ndom[i] == 0) {
+    if (on && part[i] && rank[i] < 0 && ndom[i] == 0) {
       infront[i] = 1;
       atomicAdd(&cnt, 1);
     }
@@ -190,19 +222,15 @@ __global__ void __launch_bounds__(NSGA_MAX) nsga_survive_kernel(const float *__r
     if (c == 0) break;
     if (on && infront[i]) rank[i] = r;
     if (i == 0) {
-      if (r_cut < 0 && cum + c >= P) { r_cut = r; need = P - cum; }
+      if (r_cut < 0 && cum + c >= Pf) { r_cut = r; need = Pf - cum; }
       cum += c;
     }
     __syncthreads();
     if (r_cut >= 0) break;
-    if (on && rank[i] < 0) {
+    if (on && part[i] && rank[i] < 0) {
       int sub = 0;
       for (int j = 0; j < N; ++j)
-        if (infront[j]) {
-          const bool le = f[j][0] <= f[i][0] && f[j][1] <= f[i][1] && f[j][2] <= f[i][2];
-          const bool lt = f[j][0] < f[i][0] || f[j][1] < f[i][1] || f[j][2] < f[i][2];
-          sub += (le && lt) ? 1 : 0;
-        }
+        if (infront[j]) sub += dominates(j) ? 1 : 0;
       ndom[i] -= sub;
     }
     __syncthreads();
@@ -217,7 +245,7 @@ __global__ void __launch_bounds__(NSGA_MAX) nsga_survive_kernel(const float *__r
   }
   __syncthreads();
   const bool mine = on && rc >= 0 && rank[i] == rc;
-  for (int k = 0; k < 3; ++k) {
+  for (int k = 0; k < K; ++k) {
     // position of i inside the cut front along objective k (counting sort, ties by index), then its neighbours
     int pos = 0, m = 0;
     float fmin = INFINITY, fmax = -INFINITY;
@@ -244,6 +272,14 @@ __global__ void __launch_bounds__(NSGA_MAX) nsga_survive_kernel(const float *__r
       if (rank[j] == rc) better += (crowd[j] > crowd[i] || (crowd[j] == crowd[i] && j < i)) ? 1 : 0;
     if (better < need) keep[i] = 1;
   }
+  // ---- the remaining P - Pf slots: the other rows by (bad, cv, merged index)
+  if (constrained && on && !part[i]) {
+    int before = 0;
+    for (int j = 0; j < N; ++j)
+      if (!part[j])
+        before += (bad[j] < bad[i] || (bad[j] == bad[i] && (cvk[j] < cvk[i] || (cvk[j] == cvk[i] && j < i)))) ? 1 : 0;
+    if (before < P - Pf) keep[i] = 1;
+  }
   __syncthreads();
   // ---- stable compaction into the next population
   if (on && keep[i]) {
@@ -252,7 +288,8 @@ __global__ void __launch_bounds__(NSGA_MAX) nsga_survive_kernel(const float *__r
     const float *src = i < P ? X + (int64_t)i * D : C + (int64_t)(i - P) * D;
     float *row = Xn + (int64_t)dst * D;
     for (int k = 0; k < D; ++k) row[k] = src[k];
-    for (int k = 0; k < 3; ++k) Fn[(int64_t)dst * 3 + k] = f[i][k];
+    for (int k = 0; k < K; ++k) Fn[(int64_t)dst * K + k] = f[i][k];
+    if (constrained) CVn[dst] = i < P ? CV[i] : CVC[i - P];
     split_row(src, d, D - d, Xcn + (int64_t)dst * d, Xen + (int64_t)dst * (D - d));
   }
 }
@@ -276,13 +313,32 @@ int launch_nsga_mate(const float *X, int64_t P, int64_t D, int64_t d, const int3
   return HB_OK;
 }
 
-int launch_nsga_survive(const float *X, const float *F, const float *C, const float *FC, int64_t P, int64_t D, int64_t d,
-                        float *Xn, float *Fn, float *Xcn, int32_t *Xen, cudaStream_t st) {
+int launch_nsga_survive_k(const float *X, const float *F, const float *CV, const float *C, const float *FC, const float *CVC,
+                          int64_t P, int64_t D, int64_t d, int K, float *Xn, float *Fn, float *CVn, float *Xcn, int32_t *Xen,
+                          cudaStream_t st) {
   if (P <= 0 || 2 * P > NSGA_MAX || D <= 0 || d < 0 || d > D) return HB_ERR_INVALID;
-  nsga_survive_kernel<<<1, NSGA_MAX, 0, st>>>(X, F, C, FC, (int)P, (int)D, (int)d, Xn, Fn, Xcn, Xen);
+  if ((CV == nullptr) != (CVC == nullptr) || (CV != nullptr && CVn == nullptr)) return HB_ERR_INVALID;
+#define HB_SURV(KK) nsga_survive_kernel<KK><<<1, NSGA_MAX, 0, st>>>(X, F, CV, C, FC, CVC, (int)P, (int)D, (int)d, Xn, Fn, CVn, Xcn, Xen)
+  switch (K) {
+    case 1: HB_SURV(1); break;
+    case 2: HB_SURV(2); break;
+    case 3: HB_SURV(3); break;
+    case 4: HB_SURV(4); break;
+    case 5: HB_SURV(5); break;
+    case 6: HB_SURV(6); break;
+    case 7: HB_SURV(7); break;
+    case 8: HB_SURV(8); break;
+    default: return HB_ERR_INVALID;
+  }
+#undef HB_SURV
   count_launches(1);
   HB_LAUNCH_CHECK("nsga_survive");
   return HB_OK;
+}
+
+int launch_nsga_survive(const float *X, const float *F, const float *C, const float *FC, int64_t P, int64_t D, int64_t d,
+                        float *Xn, float *Fn, float *Xcn, int32_t *Xen, cudaStream_t st) {
+  return launch_nsga_survive_k(X, F, nullptr, C, FC, nullptr, P, D, d, 3, Xn, Fn, nullptr, Xcn, Xen, st);
 }
 
 }  // namespace hb

@@ -1,15 +1,22 @@
-// 3-objective non-dominated filter (all objectives minimised): the rank-0 set that pymoo's NSGA-II hands back
-// as res.X in HEBO/hebo/acq_optimizers/evolution_optimizer.py:141-149, computed exactly on the device for
-// candidate batches of any size.
+// K-objective constrained non-dominated filter (all objectives minimised, 1 <= K <= 8): the rank-0 set that pymoo's NSGA-II
+// hands back as res.X in HEBO/hebo/acq_optimizers/evolution_optimizer.py:141-149, computed exactly on the device for
+// candidate batches of any size.  F is read with a row stride ldf >= K, so the objective columns of a wider [m, O]
+// acquisition output (GeneralAcq: objectives first, then constraints) are filtered in place.
 //
 //   a dominates b  <=>  all(a <= b) and any(a < b)
 // A row with a NaN objective never dominates (every comparison is false) and is EXCLUDED from the front: it cannot be
 // dominated either, and the selection step (hebo.py:182-193) must never be handed a candidate whose acquisition is NaN.
+// With a constraint violation cv [m] (cv = sum_j max(0, g_j), pymoo 0.6 calc_cv as recalled -- pymoo is not installed)
+// only FEASIBLE rows (cv <= 0; a NaN cv is never feasible) take part: an infeasible row is loaded as NaN, so it neither
+// dominates nor survives.  If no row is feasible, the result is the single row of least cv (lowest index on ties, rows
+// with a NaN objective or cv never chosen) -- the least_infeasible rule of pymoo's filter_optimum behind res.X -- found
+// with one 64-bit atomicMin on the device, without a host read.
 //
 // m <= 4096: one tiled all-pairs pass.  Larger m: (1) exact front FS of a stratified sample (strided_row), (2) every point is
 // tested against FS only (anything FS dominates is dominated in the full set), (3) exact all-pairs among the
-// survivors.  By transitivity of dominance step 3 sees every true dominator, so the result is exact.
-// Compaction is order preserving (count / scan / scatter), so idx_out is ascending and deterministic.
+// survivors.  By transitivity of dominance (restricted to the feasible rows, for any K) step 3 sees every true dominator,
+// so the result is exact.  Compaction is order preserving (count / scan / scatter), so idx_out is ascending and
+// deterministic.  hb_pareto_front3 is the K = 3, ldf = 3, cv = NULL instantiation of this one code path.
 #include "kernels.h"
 
 namespace hb {
@@ -29,17 +36,19 @@ __device__ __forceinline__ int64_t strided_row(int a, int stride) {
   return (int64_t)a * stride + (int64_t)(h % (uint32_t)stride);
 }
 
-// flags[a] := 0 if list-A element a is dominated by an element of list B (or carries a NaN); flags must be preset to 1.
-// idxA / idxB == nullptr -> identity lists of length *nA / *nB (or the host bounds when the count pointers are null).
-// gridDim.y splits list B into segments (each block tests its 256 A rows against one segment and only ever CLEARS flags:
-// idempotent, no ordering needed), so a short list A against a long list B -- the 4096 x 4096 sample-front pass, 16 blocks
-// and 205 us when B was walked by one block per A tile -- still fills the machine.
-__global__ void __launch_bounds__(PB) nondominated_kernel(const float *__restrict__ F, const int32_t *__restrict__ idxA,
+// flags[a] := 0 if list-A element a is dominated by an element of list B (or carries a NaN, or is infeasible); flags must be
+// preset to 1.  idxA / idxB == nullptr -> identity lists of length *nA / *nB (or the host bounds when the count pointers are
+// null).  gridDim.y splits list B into segments (each block tests its 256 A rows against one segment and only ever CLEARS
+// flags: idempotent, no ordering needed), so a short list A against a long list B -- the 4096 x 4096 sample-front pass, 16
+// blocks and 205 us when B was walked by one block per A tile -- still fills the machine.
+template <int K>
+__global__ void __launch_bounds__(PB) nondominated_kernel(const float *__restrict__ F, int64_t ldf, const float *__restrict__ cv,
+                                                          const int32_t *__restrict__ idxA,
                                                           const int32_t *__restrict__ nA_ptr, int nA_host, int strideA,
                                                           const int32_t *__restrict__ idxB,
                                                           const int32_t *__restrict__ nB_ptr, int nB_host, int strideB,
                                                           uint8_t *__restrict__ flags) {
-  __shared__ float b0[PB], b1[PB], b2[PB];
+  __shared__ float bs[K][PB];
   const int nA = nA_ptr ? *nA_ptr : nA_host;
   const int nB = nB_ptr ? *nB_ptr : nB_host;
   if ((int)(blockIdx.x * PB) >= nA) return;
@@ -47,29 +56,38 @@ __global__ void __launch_bounds__(PB) nondominated_kernel(const float *__restric
   const int jbeg = blockIdx.y * seg, jend = min(nB, jbeg + seg);
   const int a = blockIdx.x * PB + threadIdx.x;
   const bool active = a < nA;
-  float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+  float av[K];
+  bool dominated = !active;
+#pragma unroll
+  for (int k = 0; k < K; ++k) av[k] = 0.f;
   if (active) {
     const int64_t ia = idxA ? idxA[a] : strided_row(a, strideA);
-    a0 = F[ia * 3 + 0];
-    a1 = F[ia * 3 + 1];
-    a2 = F[ia * 3 + 2];
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      av[k] = F[ia * ldf + k];
+      dominated |= isnan(av[k]);
+    }
+    if (cv) dominated |= !(cv[ia] <= 0.f);
   }
-  bool dominated = !active || isnan(a0) || isnan(a1) || isnan(a2);
   for (int j0 = jbeg; j0 < jend; j0 += PB) {
     const int j = j0 + threadIdx.x;
     if (j < jend) {
       const int64_t ib = idxB ? idxB[j] : strided_row(j, strideB);
-      b0[threadIdx.x] = F[ib * 3 + 0];
-      b1[threadIdx.x] = F[ib * 3 + 1];
-      b2[threadIdx.x] = F[ib * 3 + 2];
+      const bool feasible = !cv || cv[ib] <= 0.f;
+#pragma unroll
+      for (int k = 0; k < K; ++k) bs[k][threadIdx.x] = feasible ? F[ib * ldf + k] : NAN;
     }
     __syncthreads();
     const int lim = min(PB, jend - j0);
     if (!dominated) {
       for (int u = 0; u < lim; ++u) {
-        const float x0 = b0[u], x1 = b1[u], x2 = b2[u];
-        const bool le = (x0 <= a0) & (x1 <= a1) & (x2 <= a2);
-        const bool lt = (x0 < a0) | (x1 < a1) | (x2 < a2);
+        bool le = true, lt = false;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+          const float x = bs[k][u];
+          le &= x <= av[k];
+          lt |= x < av[k];
+        }
         if (le & lt) {
           dominated = true;
           break;
@@ -79,6 +97,34 @@ __global__ void __launch_bounds__(PB) nondominated_kernel(const float *__restric
     if (__syncthreads_and(dominated)) break;
   }
   if (active && dominated) flags[a] = 0;
+}
+
+// least-infeasible candidate: key = (float bits of cv) << 32 | row, over the rows without a NaN objective or cv (cv >= 0 as
+// a sum of max(0, g), so the float bits order like the values)
+template <int K>
+__global__ void __launch_bounds__(PB) least_cv_kernel(const float *__restrict__ F, int64_t ldf, const float *__restrict__ cv,
+                                                      int m, unsigned long long *__restrict__ key) {
+  const int r = blockIdx.x * PB + threadIdx.x;
+  unsigned long long mine = ~0ull;
+  if (r < m) {
+    const float c = cv[r];
+    bool ok = !isnan(c);
+#pragma unroll
+    for (int k = 0; k < K; ++k) ok &= !isnan(F[(int64_t)r * ldf + k]);
+    if (ok) mine = ((unsigned long long)__float_as_uint(fmaxf(c, 0.0f)) << 32) | (unsigned)r;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mine = min(mine, __shfl_xor_sync(0xffffffffu, mine, o));
+  if ((threadIdx.x & 31) == 0 && mine != ~0ull) atomicMin(key, mine);
+}
+
+// no feasible row -> the front is the least-infeasible row
+__global__ void least_cv_apply_kernel(const unsigned long long *__restrict__ key, int32_t *__restrict__ idx_out,
+                                      int32_t *__restrict__ count) {
+  if (*count == 0 && *key != ~0ull) {
+    idx_out[0] = (int32_t)(*key & 0xffffffffull);
+    *count = 1;
+  }
 }
 
 // order-preserving compaction of list A by flags: count -> scan -> scatter
@@ -148,6 +194,7 @@ struct ParetoWs {
   int32_t *listS;    // sample front
   int32_t *nS;
   int32_t *nA;
+  unsigned long long *key;   // least-infeasible row (inside the nS slot's padding)
 };
 
 static ParetoWs carve_pareto(void *ws, int64_t m) {
@@ -160,6 +207,7 @@ static ParetoWs carve_pareto(void *ws, int64_t m) {
   w.listS = (int32_t *)p;         p += round_up((int64_t)PARETO_SAMPLE * 4, 256);
   w.nS = (int32_t *)p;            p += 256;
   w.nA = (int32_t *)p;            p += 256;
+  w.key = reinterpret_cast<unsigned long long *>(w.nS + 32);
   return w;
 }
 
@@ -176,8 +224,9 @@ static void compact(const uint8_t *flags, const int32_t *idxA, const int32_t *nA
   compact_scatter_kernel<<<nblocks, PB, 0, st>>>(flags, idxA, nA_ptr, nA_host, strideA, counts, out_idx);
 }
 
-int launch_pareto3(const float *F, int64_t m, int32_t *idx_out, int32_t *count, void *ws, int64_t ws_bytes,
-                   cudaStream_t st) {
+template <int K>
+static int pareto_impl(const float *F, int64_t m, int64_t ldf, const float *cv, int32_t *idx_out, int32_t *count, void *ws,
+                       int64_t ws_bytes, cudaStream_t st) {
   if (m <= 0 || m > 0x7fffffff) return HB_ERR_INVALID;
   if ((size_t)ws_bytes < pareto_ws_bytes(m)) return HB_ERR_INVALID;
   ParetoWs w = carve_pareto(ws, m);
@@ -191,7 +240,7 @@ int launch_pareto3(const float *F, int64_t m, int32_t *idx_out, int32_t *count, 
   };
   if (mi <= PARETO_DIRECT_MAX) {
     HB_CUDA(cudaMemsetAsync(w.flags, 1, (size_t)mi, st));
-    nondominated_kernel<<<dim3((unsigned)ceil_div(mi, PB), (unsigned)segs(mi, mi)), PB, 0, st>>>(F, nullptr, nullptr, mi, 1, nullptr, nullptr, mi, 1, w.flags);
+    nondominated_kernel<K><<<dim3((unsigned)ceil_div(mi, PB), (unsigned)segs(mi, mi)), PB, 0, st>>>(F, ldf, cv, nullptr, nullptr, mi, 1, nullptr, nullptr, mi, 1, w.flags);
     compact(w.flags, nullptr, nullptr, mi, 1, w.counts, idx_out, count, st);
     count_launches(4);
   } else {
@@ -199,21 +248,48 @@ int launch_pareto3(const float *F, int64_t m, int32_t *idx_out, int32_t *count, 
     const int stride = (int)(m / PARETO_SAMPLE);
     const int ns = PARETO_SAMPLE;
     HB_CUDA(cudaMemsetAsync(w.flags, 1, (size_t)ns, st));
-    nondominated_kernel<<<dim3((unsigned)ceil_div(ns, PB), (unsigned)segs(ns, ns)), PB, 0, st>>>(F, nullptr, nullptr, ns, stride, nullptr, nullptr, ns, stride, w.flags);
+    nondominated_kernel<K><<<dim3((unsigned)ceil_div(ns, PB), (unsigned)segs(ns, ns)), PB, 0, st>>>(F, ldf, cv, nullptr, nullptr, ns, stride, nullptr, nullptr, ns, stride, w.flags);
     compact(w.flags, nullptr, nullptr, ns, stride, w.counts, w.listS, w.nS, st);
     // (2) all points against the sample front (a short list: one segment)
     HB_CUDA(cudaMemsetAsync(w.flags, 1, (size_t)mi, st));
-    nondominated_kernel<<<(int)ceil_div(mi, PB), PB, 0, st>>>(F, nullptr, nullptr, mi, 1, w.listS, w.nS, 0, 1, w.flags);
+    nondominated_kernel<K><<<(int)ceil_div(mi, PB), PB, 0, st>>>(F, ldf, cv, nullptr, nullptr, mi, 1, w.listS, w.nS, 0, 1, w.flags);
     compact(w.flags, nullptr, nullptr, mi, 1, w.counts, w.listA, w.nA, st);
     // (3) exact all-pairs among the survivors (count known only on the device: launch for the upper bound; blocks past the
     //     count exit at once; four B segments keep a long survivor list from serialising on a few SMs)
     HB_CUDA(cudaMemsetAsync(w.flags, 1, (size_t)mi, st));
-    nondominated_kernel<<<dim3((unsigned)ceil_div(mi, PB), 4), PB, 0, st>>>(F, w.listA, w.nA, 0, 1, w.listA, w.nA, 0, 1, w.flags);
+    nondominated_kernel<K><<<dim3((unsigned)ceil_div(mi, PB), 4), PB, 0, st>>>(F, ldf, cv, w.listA, w.nA, 0, 1, w.listA, w.nA, 0, 1, w.flags);
     compact(w.flags, w.listA, w.nA, mi, 1, w.counts, idx_out, count, st);
     count_launches(12);
   }
-  HB_LAUNCH_CHECK("pareto3");
+  if (cv) {
+    HB_CUDA(cudaMemsetAsync(w.key, 0xff, sizeof(unsigned long long), st));
+    least_cv_kernel<K><<<(int)ceil_div(mi, PB), PB, 0, st>>>(F, ldf, cv, mi, w.key);
+    least_cv_apply_kernel<<<1, 1, 0, st>>>(w.key, idx_out, count);
+    count_launches(2);
+  }
+  HB_LAUNCH_CHECK("pareto");
   return HB_OK;
+}
+
+int launch_pareto(const float *F, int64_t m, int K, int64_t ldf, const float *cv, int32_t *idx_out, int32_t *count, void *ws,
+                  int64_t ws_bytes, cudaStream_t st) {
+  if (ldf < K) return HB_ERR_INVALID;
+  switch (K) {
+    case 1: return pareto_impl<1>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 2: return pareto_impl<2>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 3: return pareto_impl<3>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 4: return pareto_impl<4>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 5: return pareto_impl<5>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 6: return pareto_impl<6>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 7: return pareto_impl<7>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    case 8: return pareto_impl<8>(F, m, ldf, cv, idx_out, count, ws, ws_bytes, st);
+    default: return HB_ERR_INVALID;
+  }
+}
+
+int launch_pareto3(const float *F, int64_t m, int32_t *idx_out, int32_t *count, void *ws, int64_t ws_bytes,
+                   cudaStream_t st) {
+  return launch_pareto(F, m, 3, 3, nullptr, idx_out, count, ws, ws_bytes, st);
 }
 
 // ================================================================================= multi-GPU front exchange

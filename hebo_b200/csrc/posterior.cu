@@ -387,6 +387,71 @@ __global__ void __launch_bounds__(256) mace_kernel(const float *__restrict__ mup
   F[gr * 3 + 2] = o2;
 }
 
+// ---- GeneralAcq.eval (acq.py:233-242) over O = num_obj + num_constr outputs, fp32, the reference's operation order:
+//   ps = sqrt(ps2).clamp(min = eps) ; py += sqrt(noise) * xi (use_noise) ; out = py - kappa ps (objectives) | - c_kappa ps
+// mu / var [O, m] output-major (O calls of the posterior, one output row each); out [m, O] row-major like the reference's
+// `out`; cv [m] (optional) = sum_j max(0, out[:, num_obj + j]) in ascending j, pymoo 0.6 calc_cv as recalled (NaN
+// propagates).  xi [m, O] = the reference's single torch.randn(py.shape) draw, or NULL: Philox normals keyed by
+// (seed, rng_offset + row, output), the pair (2 j, 2 j + 1) from counter word j -- with O <= 2 the draws of mace_kernel.
+__device__ __forceinline__ void philox_normal2_word(uint64_t seed, uint64_t row, uint32_t word, float &z0, float &z1) {
+  uint32_t c[4] = {(uint32_t)row, (uint32_t)(row >> 32), word, 0u};
+  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    philox_round(c, k0, k1);
+    k0 += 0x9E3779B9u;
+    k1 += 0xBB67AE85u;
+  }
+  const float u0 = ((float)c[0] + 0.5f) * 2.3283064365386963e-10f;   // (0,1)
+  const float u1 = ((float)c[1] + 0.5f) * 2.3283064365386963e-10f;
+  const float rad = sqrtf(-2.0f * logf(u0));
+  float sn, cs;
+  sincospif(2.0f * u1, &sn, &cs);
+  z0 = rad * cs;
+  z1 = rad * sn;
+}
+
+__global__ void __launch_bounds__(256) general_acq_kernel(const float *__restrict__ mu, const float *__restrict__ var, int64_t m,
+                                                          int num_obj, int O, const float *__restrict__ noise_var, float kappa,
+                                                          float c_kappa, int use_noise, const float *__restrict__ xi,
+                                                          uint64_t seed, int64_t rng_offset, float *__restrict__ out,
+                                                          float *__restrict__ cv) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= m) return;
+  float cvs = 0.0f, z1 = 0.0f;
+  for (int o = 0; o < O; ++o) {
+    float py = mu[(int64_t)o * m + r];
+    const float s = sqrtf(var[(int64_t)o * m + r]);
+    const float ps = isnan(s) ? s : fmaxf(s, 1.1920929e-07f);                // clamp(min = finfo.eps) keeps a NaN
+    if (use_noise) {
+      float z;
+      if (xi) {
+        z = xi[r * O + o];
+      } else if ((o & 1) == 0) {
+        philox_normal2_word(seed, (uint64_t)(rng_offset + r), (uint32_t)(o >> 1), z, z1);
+      } else {
+        z = z1;
+      }
+      py = __fadd_rn(py, __fmul_rn(sqrtf(noise_var[o]), z));                  // acq.py:236-238
+    }
+    const float v = __fsub_rn(py, __fmul_rn(o < num_obj ? kappa : c_kappa, ps));   // acq.py:240-241
+    out[r * O + o] = v;
+    if (o >= num_obj) cvs = __fadd_rn(cvs, v > 0.0f ? v : (isnan(v) ? v : 0.0f));
+  }
+  if (cv) cv[r] = cvs;
+}
+
+int launch_general_acq(const float *mu, const float *var, int64_t m, int num_obj, int num_constr, const float *noise_var,
+                       float kappa, float c_kappa, int use_noise, const float *xi, uint64_t seed, int64_t rng_offset, float *out,
+                       float *cv, cudaStream_t st) {
+  if (m <= 0 || num_obj < 1 || num_obj > 8 || num_constr < 0 || num_obj + num_constr > 64) return HB_ERR_INVALID;
+  general_acq_kernel<<<(int)ceil_div(m, 256), 256, 0, st>>>(mu, var, m, num_obj, num_obj + num_constr, noise_var, kappa, c_kappa,
+                                                            use_noise, xi, seed, rng_offset, out, cv);
+  count_launches(1);
+  HB_LAUNCH_CHECK("general_acq");
+  return HB_OK;
+}
+
 int kstar_groups(int64_t np) { return (int)ceil_div(np, KS_GROUP); }
 
 // plain fp32 K* rows + mean partials (posterior_grad.cu)

@@ -82,6 +82,67 @@ def rank_and_crowding_survival(F: np.ndarray, n_survive: int) -> np.ndarray:
     return np.asarray(keep, dtype=np.int64)
 
 
+def constraint_violation(G: np.ndarray) -> np.ndarray:
+    """cv = sum_j max(0, g_j) per row (pymoo 0.6 calc_cv as recalled; pymoo is not installed).  A NaN propagates."""
+    G = np.asarray(G)
+    return np.where(np.isnan(G), G, np.maximum(G, 0)).sum(1) if G.shape[1] else np.zeros(G.shape[0], dtype=G.dtype)
+
+
+def constrained_front(F: np.ndarray, cv: Optional[np.ndarray] = None) -> np.ndarray:
+    """Ascending indices of the non-dominated FEASIBLE rows of F [m, K] (cv <= 0; a NaN objective or cv excludes a row).
+    With no feasible row: the single row of least cv, lowest index on ties (pymoo's filter_optimum(least_infeasible=True)
+    behind res.X, as recalled).  The host restatement of hb_pareto_front."""
+    F = np.asarray(F, dtype=np.float64)
+    m = F.shape[0]
+    ok = ~np.isnan(F).any(1)
+    if cv is not None:
+        cv = np.asarray(cv, dtype=np.float64).reshape(-1)
+        ok &= ~np.isnan(cv)
+    feas = ok & (cv <= 0) if cv is not None else ok
+    idx = np.flatnonzero(feas)
+    if idx.size:
+        # rows in ascending objective sum (a dominator's sum is smaller), in blocks: each row is tested against the front
+        # found so far and against its own block
+        order = idx[np.argsort(F[idx].sum(1), kind="stable")]
+        front = np.zeros(0, dtype=np.int64)
+        for b in range(0, order.size, 1024):
+            blk = order[b:b + 1024]
+            Fb = F[blk]
+            dom = np.zeros(blk.size, dtype=bool)
+            for f0 in range(0, front.size, 1024):
+                Ff = F[front[f0:f0 + 1024]]
+                dom |= ((Ff[:, None, :] <= Fb[None]).all(-1) & (Ff[:, None, :] < Fb[None]).any(-1)).any(0)
+            blk = blk[~dom]                                  # (a block row the front dominates dominates nothing new)
+            front = np.concatenate([front, blk[~dominance_matrix(F[blk]).any(0)]])
+        return np.sort(front)
+    if cv is None or not ok.any():
+        return np.zeros(0, dtype=np.int64)
+    cand = np.flatnonzero(ok)
+    return cand[[int(np.argmin(np.maximum(cv[cand], 0)))]]                 # argmin: first of the ties
+
+
+def constrained_rank_and_crowding_survival(F: np.ndarray, cv: Optional[np.ndarray], n_survive: int) -> np.ndarray:
+    """Survivors of the merged population under pymoo's filter_infeasible rule (Survival.do, as recalled): feasible rows
+    (cv <= 0, finite objectives) by rank-and-crowding for min(n_feasible, n_survive) slots, then the other rows in
+    ascending cv (lower index first), rows with a non-finite objective or a NaN cv last.  Ascending indices.  Without cv: the
+    unconstrained survival with every non-finite row at +inf.  The host restatement of hb_nsga2_survive_k."""
+    F = np.asarray(F, dtype=np.float64)
+    finite = np.isfinite(F).all(1)
+    Fi = np.where(finite[:, None], F, np.inf)
+    if cv is None:
+        return np.sort(rank_and_crowding_survival(Fi, n_survive))
+    cv = np.asarray(cv, dtype=np.float64).reshape(-1)
+    bad = ~finite | np.isnan(cv)
+    feas = ~bad & (cv <= 0)
+    fi = np.flatnonzero(feas)
+    keep = fi[rank_and_crowding_survival(Fi[fi], min(fi.size, n_survive))].tolist() if fi.size else []
+    rest = np.flatnonzero(~feas)
+    key = np.where(bad[rest], 0.0, cv[rest])
+    order = np.lexsort((rest, key, bad[rest]))                              # (bad, cv, index)
+    keep += rest[order[: n_survive - len(keep)]].tolist()
+    return np.sort(np.asarray(keep, dtype=np.int64))
+
+
 class EvolutionOpt:
     def __init__(self, lb, ub, acq_fn: Callable[[np.ndarray], np.ndarray], pop: int = 100, iters: int = 100,
                  seed: Optional[int] = None, sbx_eta: float = 15.0, sbx_prob: float = 0.9, sbx_prob_var: float = 0.5,
@@ -185,18 +246,22 @@ class EvolutionOpt:
 
 
 class DeviceNSGA2:
-    """NSGA-II over the MACE objectives with the population resident on the GPU (include/hebo_b200.h "device NSGA-II").
+    """NSGA-II with the population resident on the GPU (include/hebo_b200.h "device NSGA-II").
 
     kinds [D]: 'real' | 'int' | 'choice' per optimisation column (numeric columns first, then the categorical ones:
     evolution_optimizer.py:26-41); lb / ub [D]; fixed: {column index: value} (fix_input, :97-101).  `score(Xc, Xe, gen)`
-    returns the objectives F [pop, 3] of a batch as a device tensor (the fused posterior + MACE call)."""
+    returns the objectives F [pop, num_obj] of a batch as a device tensor (the fused posterior + MACE call for the default
+    num_obj = 3), or a pair (F, cv) with the constraint violation cv [pop] (GeneralAcq): survival then follows pymoo's
+    filter_infeasible rule and the result is the constrained front (hb_nsga2_survive_k, hb_pareto_front)."""
 
     KIND = {"real": 0, "int": 1, "choice": 2}
 
     def __init__(self, kinds, lb, ub, num_numeric: int, score: Callable, pop: int = 100, iters: int = 100,
-                 seed: Optional[int] = None, fixed: Optional[dict] = None, device="cuda"):
+                 seed: Optional[int] = None, fixed: Optional[dict] = None, device="cuda", num_obj: int = 3):
         import torch
         self.torch = torch
+        self.num_obj = int(num_obj)
+        assert 1 <= self.num_obj <= 8
         self.D, self.d, self.pop, self.iters = len(kinds), int(num_numeric), int(pop), int(iters)
         assert 2 * self.pop <= 512 and self.pop >= 2
         dev = torch.device(device)
@@ -218,11 +283,12 @@ class DeviceNSGA2:
                 t.empty(P, D - d, dtype=t.int32, device=dev))
 
     def optimize(self, initial_suggest=None):
-        """Returns (Xc [K, d] fp32, Xe [K, e] int32, F [K, 3]) of the non-dominated members of the final population
-        (res.X of evolution_optimizer.py:141-149), all on the device."""
+        """Returns (Xc [K, d] fp32, Xe [K, e] int32, F [K, num_obj]) of the non-dominated members of the final population
+        (res.X of evolution_optimizer.py:141-149; with constraints the feasible front, or the least-infeasible member when
+        none is feasible), all on the device.  With constraints `self.pop_cv` holds the final population's cv."""
         from . import _lib
         from .pareto import pareto_front
-        t, lib, P, D, d = self.torch, _lib.lib(), self.pop, self.D, self.d
+        t, lib, P, D, d, K = self.torch, _lib.lib(), self.pop, self.D, self.d, self.num_obj
         st = _lib.stream_ptr
         X, Xc, Xe = self._bufs()
         Xn, Xcn, Xen = self._bufs()
@@ -230,20 +296,33 @@ class DeviceNSGA2:
         init = None if initial_suggest is None else t.as_tensor(np.asarray(initial_suggest, dtype=np.float32).reshape(-1, D)).to(self.dev)
         n_init = 0 if init is None else min(init.shape[0], P)
         pc = lambda x: _lib.ptr(x) if x.numel() else None
+
+        def scored(xc, xe, gen):
+            out = self.score(xc, xe, gen)
+            F, cv = out if isinstance(out, tuple) else (out, None)
+            F = F.contiguous()
+            assert F.shape[1] == K, f"score returned {F.shape[1]} objectives, expected {K}"
+            return F, (None if cv is None else cv.reshape(-1).contiguous())
         with t.cuda.device(self.dev):
             _lib.check(lib.hb_nsga2_init(_lib.ptr(X), P, D, d, _lib.ptr(self.kind), _lib.ptr(self.lb), _lib.ptr(self.ub), _lib.ptr(self.fixed),
                                          _lib.ptr(init), n_init, self.seed, pc(Xc), pc(Xe), st()), "hb_nsga2_init")
-            F = self.score(Xc, Xe, 0).contiguous()
+            F, cv = scored(Xc, Xe, 0)
             Fn = t.empty_like(F)
+            cvn = None if cv is None else t.empty_like(cv)
             self.n_evals = P
             for gen in range(1, self.iters):                       # ('n_gen', iters): generation 1 is the initial population
                 _lib.check(lib.hb_nsga2_mate(_lib.ptr(X), P, D, d, _lib.ptr(self.kind), _lib.ptr(self.lb), _lib.ptr(self.ub),
                                              _lib.ptr(self.fixed), self.seed, gen, _lib.ptr(C), pc(Cc), pc(Ce), st()), "hb_nsga2_mate")
-                FC = self.score(Cc, Ce, gen).contiguous()
-                _lib.check(lib.hb_nsga2_survive(_lib.ptr(X), _lib.ptr(F), _lib.ptr(C), _lib.ptr(FC), P, D, d, _lib.ptr(Xn), _lib.ptr(Fn),
-                                                pc(Xcn), pc(Xen), st()), "hb_nsga2_survive")
-                X, Xn, Xc, Xcn, Xe, Xen, F, Fn = Xn, X, Xcn, Xc, Xen, Xe, Fn, F
+                FC, cvc = scored(Cc, Ce, gen)
+                if K == 3 and cv is None:                          # the MACE path
+                    _lib.check(lib.hb_nsga2_survive(_lib.ptr(X), _lib.ptr(F), _lib.ptr(C), _lib.ptr(FC), P, D, d, _lib.ptr(Xn), _lib.ptr(Fn),
+                                                    pc(Xcn), pc(Xen), st()), "hb_nsga2_survive")
+                else:
+                    _lib.check(lib.hb_nsga2_survive_k(_lib.ptr(X), _lib.ptr(F), _lib.ptr(cv), _lib.ptr(C), _lib.ptr(FC), _lib.ptr(cvc), P, D, d,
+                                                      K, _lib.ptr(Xn), _lib.ptr(Fn), _lib.ptr(cvn), pc(Xcn), pc(Xen), st()),
+                               "hb_nsga2_survive_k")
+                X, Xn, Xc, Xcn, Xe, Xen, F, Fn, cv, cvn = Xn, X, Xcn, Xc, Xen, Xe, Fn, F, cvn, cv
                 self.n_evals += P
-        self.pop_X, self.pop_F = X, F
-        idx = pareto_front(F)
+        self.pop_X, self.pop_F, self.pop_cv = X, F, cv
+        idx = pareto_front(F, cv)
         return Xc[idx], Xe[idx], F[idx]

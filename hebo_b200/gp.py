@@ -488,7 +488,10 @@ class GP(BaseModel):
         return self._side_stream
 
     def _posterior(self, Xs_dev: Optional[torch.Tensor], want_F: bool, tau=0.0, kappa=0.0, eps=0.0, xi1=None, xi2=None,
-                   seed: int = 0, want_mu_var: bool = True, Xe_dev: Optional[torch.Tensor] = None):
+                   seed: int = 0, want_mu_var: bool = True, Xe_dev: Optional[torch.Tensor] = None,
+                   out_mu: Optional[torch.Tensor] = None, out_var: Optional[torch.Tensor] = None):
+        """out_mu / out_var: optional contiguous fp32 device rows [m] to write the posterior into (GeneralAcq stacks the
+        outputs of a MultiTaskModel into one [O, m] buffer this way)."""
         lib = _lib.lib()
         assert self._fitted or hasattr(self, "Linv_dev"), "fit() first"
         # a pinned host batch larger than one chunk is uploaded chunk by chunk under the scoring (same results)
@@ -503,14 +506,15 @@ class GP(BaseModel):
             return (torch.empty(0, 3, dtype=torch.float32, device=dev) if want_F else None,
                     e if want_mu_var else None, e.clone() if want_mu_var else None)
         F = torch.empty(m, 3, dtype=torch.float32, device=dev) if want_F else None
-        mu = torch.empty(m, dtype=torch.float32, device=dev) if want_mu_var else None
-        var = torch.empty(m, dtype=torch.float32, device=dev) if want_mu_var else None
+        mu = (torch.empty(m, dtype=torch.float32, device=dev) if out_mu is None else out_mu) if want_mu_var else None
+        var = (torch.empty(m, dtype=torch.float32, device=dev) if out_var is None else out_var) if want_mu_var else None
         if self._fit_failed:
             # gp.py:152-154: "jitter is too large, output random predictions" = N(0, I) in the standardised space, pushed
             # through the same un-scaling and (for F) the MACE epilogue kernel -- never the leftovers of a failed factorisation
             print("jitter is too large, output random predictions")
-            mu_f = torch.full((m,), self._y_mean, dtype=torch.float32, device=dev)
-            var_f = torch.full((m,), max(self._y_std ** 2, EPS32), dtype=torch.float32, device=dev)
+            mu_f = torch.full((m,), self._y_mean, dtype=torch.float32, device=dev) if out_mu is None else out_mu.fill_(self._y_mean)
+            var_f = (torch.full((m,), max(self._y_std ** 2, EPS32), dtype=torch.float32, device=dev) if out_var is None
+                     else out_var.fill_(max(self._y_std ** 2, EPS32)))
             if want_F:
                 with torch.cuda.device(dev):
                     _lib.check(lib.hb_mace_epilogue(_lib.ptr(mu_f), _lib.ptr(var_f), m, float(self.noise[0]), float(tau), float(kappa),

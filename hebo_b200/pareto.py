@@ -1,11 +1,13 @@
-"""Device non-dominated filter (3 objectives, minimised) through the C ABI.
+"""Device non-dominated filter (K <= 8 objectives, minimised, optionally constrained) through the C ABI.
 
 Replaces the rank-0 extraction NSGA-II performs on the final population
-(HEBO/hebo/acq_optimizers/evolution_optimizer.py:141-149) for candidate batches of any size.
+(HEBO/hebo/acq_optimizers/evolution_optimizer.py:141-149) for candidate batches of any size; with a constraint violation
+``cv`` only feasible rows (cv <= 0) form the front, and with none feasible the least-infeasible row is returned
+(GeneralBO, HEBO/hebo/optimizers/general.py:23-204).
 """
 from __future__ import annotations
 
-from typing import Tuple
+from typing import Optional, Tuple
 
 import torch
 
@@ -23,28 +25,41 @@ def _workspace(dev: torch.device, need: int, tag: str = "front") -> torch.Tensor
     return ws
 
 
-def pareto_front_device(F: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-    """F [m,3] float32 CUDA tensor -> (idx int32 [m] whose first `count` entries are the ascending indices of the
-    non-dominated rows, count int32 [1]), both on the device; NO host synchronisation."""
+def pareto_front_device(F: torch.Tensor, cv: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """F [m, K] float32 CUDA tensor (1 <= K <= 8; a column slice of a wider row-major tensor is read in place), cv [m] or
+    None -> (idx int32 [m] whose first `count` entries are the ascending indices of the non-dominated feasible rows -- or
+    the single least-infeasible row when none is feasible -- count int32 [1]), both on the device; NO host
+    synchronisation."""
     lib = _lib.lib()
-    assert F.is_cuda and F.dim() == 2 and F.shape[1] == 3
-    F = F.to(torch.float32).contiguous()
-    m = F.shape[0]
+    assert F.is_cuda and F.dim() == 2 and 1 <= F.shape[1] <= 8
+    m, K = F.shape
     dev = F.device
     ws = _workspace(dev, int(lib.hb_pareto_workspace_bytes(m)))
     idx = torch.empty(m, dtype=torch.int32, device=dev)
     cnt = torch.zeros(1, dtype=torch.int32, device=dev)
+    if K == 3 and cv is None:                  # the 3-objective MACE front
+        F = F.to(torch.float32).contiguous()
+        with torch.cuda.device(dev):
+            st = lib.hb_pareto_front3(_lib.ptr(F), m, _lib.ptr(idx), _lib.ptr(cnt), _lib.ptr(ws), ws.numel(),
+                                      _lib.stream_ptr())
+        _lib.check(st, "hb_pareto_front3")
+        return idx, cnt
+    if F.dtype != torch.float32 or F.stride(1) != 1 or F.stride(0) < K:
+        F = F.to(torch.float32).contiguous()
+    if cv is not None:
+        assert cv.is_cuda and cv.numel() == m
+        cv = cv.reshape(-1).to(torch.float32).contiguous()
     with torch.cuda.device(dev):
-        st = lib.hb_pareto_front3(_lib.ptr(F), m, _lib.ptr(idx), _lib.ptr(cnt), _lib.ptr(ws), ws.numel(),
-                                  _lib.stream_ptr())
-    _lib.check(st, "hb_pareto_front3")
+        st = lib.hb_pareto_front(_lib.ptr(F), m, K, F.stride(0) if m else K, _lib.ptr(cv), _lib.ptr(idx), _lib.ptr(cnt),
+                                 _lib.ptr(ws), ws.numel(), _lib.stream_ptr())
+    _lib.check(st, "hb_pareto_front")
     return idx, cnt
 
 
-def pareto_front(F: torch.Tensor) -> torch.Tensor:
-    """F [m,3] float32 CUDA tensor -> ascending int64 indices (on the device) of the non-dominated rows
-    (one host read of the count)."""
-    idx, cnt = pareto_front_device(F)
+def pareto_front(F: torch.Tensor, cv: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """F [m, K] float32 CUDA tensor (and optional cv [m]) -> ascending int64 indices (on the device) of the non-dominated
+    feasible rows (one host read of the count)."""
+    idx, cnt = pareto_front_device(F, cv)
     return idx[:int(cnt.item())].to(torch.int64)
 
 

@@ -267,6 +267,27 @@ int32_t hb_sample_y(const float *Xs, const int32_t *Xe_s, int64_t m, int64_t n, 
 int32_t hb_mace_epilogue(const float *mu, const float *var, int64_t m, float noise_var, float tau, float kappa,
                          float eps, const float *xi1, const float *xi2, uint64_t seed, float *F, void *stream);
 
+/* ---- GeneralAcq epilogue  (GeneralAcq.eval, acquisitions/acq.py:233-242, over any multi-output model's predict output;
+ * the acquisition of GeneralBO, optimizers/general.py:23-204) -------------------------------------------------------------
+ * mu, var [O, m] output-major, O = num_obj + num_constr (O calls of hb_posterior_mace_ex with F = NULL write one row each),
+ * original y units; noise_var [O] device (model.noise, read when use_noise); xi [m, O] the reference's one torch.randn(py.shape)
+ * draw, or NULL -> Philox N(0,1) keyed by (seed, rng_offset + row, output).
+ * out [m, O] = py (+ sqrt(noise) xi) - kappa ps (objective columns) | - c_kappa ps (constraint columns), ps = max(sqrt(ps2), eps);
+ * cv [m] out or NULL: sum_j max(0, out[:, num_obj + j]), the constraint violation of evolution_optimizer.py:104-105 (F / G).
+ * 1 <= num_obj <= 8, num_obj + num_constr <= 64.  One launch, no host synchronisation. */
+int32_t hb_general_acq_epilogue(const float *mu, const float *var, int64_t m, int32_t num_obj, int32_t num_constr,
+                                const float *noise_var, float kappa, float c_kappa, int32_t use_noise, const float *xi, uint64_t seed,
+                                int64_t rng_offset, float *out, float *cv, void *stream);
+
+/* ---- K-objective constrained non-dominated filter  (the rank-0 / feasible set NSGA-II returns as res.X,
+ * acq_optimizers/evolution_optimizer.py:135-149, and GeneralBO's front, optimizers/general.py:182-195) --------------------
+ * F [m, ldf] (objective columns 0..K-1 of each row, ldf >= K, 1 <= K <= 8); cv [m] or NULL.  idx_out [m] int32 ascending
+ * indices of the non-dominated FEASIBLE rows (cv <= 0); count device int32.  Rows with a NaN objective or cv are excluded.
+ * If no row is feasible the result is the one row of least cv (lowest index on ties).  ws: hb_pareto_workspace_bytes(m),
+ * enough for every K.  No host synchronisation. */
+int32_t hb_pareto_front(const float *F, int64_t m, int32_t K, int64_t ldf, const float *cv, int32_t *idx_out, int32_t *count,
+                        void *ws, int64_t ws_bytes, void *stream);
+
 /* ---- 3-objective non-dominated filter  (the rank-0 set NSGA-II returns as res.X,
  * acq_optimizers/evolution_optimizer.py:141-149) ----------------------------------------------
  * F [m,3]; idx_out [m] int32 ascending indices of the non-dominated rows; count device int32.
@@ -287,6 +308,16 @@ int32_t hb_nsga2_mate(const float *X, int64_t pop, int64_t D, int64_t d, const i
                       const float *fixed, uint64_t seed, int32_t generation, float *C, float *Cc, int32_t *Ce, void *stream);
 int32_t hb_nsga2_survive(const float *X, const float *F, const float *C, const float *FC, int64_t pop, int64_t D, int64_t d,
                          float *X_next, float *F_next, float *Xc_next, int32_t *Xe_next, void *stream);
+
+/* K-objective survival with constraints (evolution_optimizer.py:104-105 hands pymoo F [pop, K] and G; the survival replaces
+ * pymoo's rank-and-crowding with its filter_infeasible rule): F / FC [pop, K], CV / CVC [pop] constraint violations (both
+ * NULL = unconstrained).  Feasible rows (cv <= 0) go through rank-and-crowding for min(n_feasible, pop) slots; the rest go to
+ * the other rows in ascending cv (lower merged index first); duplicates and non-finite objectives only fill slots nothing
+ * else can.  Survivors in ascending merged-row order; CV_next [pop] required with CV.  1 <= K <= 8.
+ * hb_nsga2_survive == K = 3 without constraints. */
+int32_t hb_nsga2_survive_k(const float *X, const float *F, const float *CV, const float *C, const float *FC, const float *CVC,
+                           int64_t pop, int64_t D, int64_t d, int32_t K, float *X_next, float *F_next, float *CV_next,
+                           float *Xc_next, int32_t *Xe_next, void *stream);
 
 /* ---- multi-GPU front exchange  (candidate-sharded scoring, BASELINE config 5: every rank filters its shard, ONE
  * all-gather of fixed-capacity front buffers, every rank merges; no reference counterpart -- the reference is one process,

@@ -1,6 +1,7 @@
 """Small end-to-end pass for compute-sanitizer (memcheck / racecheck / synccheck): numeric + mixed fit (tile-DAG Cholesky,
 tcgen05 fit GEMMs, triangular inverse, gradient kernels, CUDA-graph epochs), refined inverse, tensor-path posterior with the
-guard (vnorm_h16 + FP32 re-contraction), MACE, Pareto front, front pack / merge, device NSGA-II.
+guard (vnorm_h16 + FP32 re-contraction), MACE, Pareto front, front pack / merge, device NSGA-II, and the multi-objective /
+constrained path (GeneralAcq epilogue, K-objective constrained front, constrained K-objective survival).
 
     compute-sanitizer --tool memcheck  python tools/sanitize_run.py
     compute-sanitizer --tool racecheck python tools/sanitize_run.py
@@ -54,5 +55,16 @@ gw = hebo_b200.GP(3, 0, 1, num_epochs=4, pred_likeli=False, warp=True)          
 gw.fit(X[:200, :3], None, y[:200])
 gw.predict(X[:64, :3], None)
 gw.sample_y(X[:32, :3], None, 3)
+mt = hebo_b200.MultiTaskModel(d, 0, 3, num_epochs=4, pred_likeli=False)           # GeneralAcq epilogue + constrained fronts
+mt.fit(X[:300], None, torch.cat([y[:300], -y[:300], y[:300] - 0.2], 1))
+gacq = hebo_b200.GeneralAcq(mt, 2, 1, kappa=2.0, c_kappa=0.5, use_noise=True)
+gout, gcv = gacq.evaluate(Xs.cuda(), None, device_out=True, return_cv=True)
+pareto_front(gout[:, :2], gcv)
+Fk = torch.randn(20000, 5, device="cuda")
+pareto_front(Fk, torch.rand(20000, device="cuda") + 0.1)                   # sieve path, nothing feasible
+evo_k = DeviceNSGA2(["real", "real", "choice"], [-1, -1, 0], [1, 1, 3], 2,
+                    lambda xc, xe, g: (torch.stack([xc[:, 0], -xc[:, 1]], 1), (xc[:, 0] + xc[:, 1]).clamp_min(0)), pop=32, iters=4,
+                    seed=2, num_obj=2)
+evo_k.optimize()
 torch.cuda.synchronize()
 print("sanitize_run ok", int(idx.numel()))
